@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mray/s of the ToyPathTracer hot path (DrawTest -> Trace/HitWorld/Scatter) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode fast|exact]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode fast|exact] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): the reference's 46-sphere scene, 1280x720, 4 spp per frame, flags = 0
 (non-progressive: every frame is a fresh image, BASELINE "DO_PROGRESSIVE off"). One STEP = one frame = one DrawTest
@@ -23,6 +23,12 @@ call of the reference (UpdateTest + DrawTest): ~16.8 M rays (camera + bounce + s
 
 --impl reference times the UNMODIFIED reference C++ path (oracle/_ref/libtoyref.so, enkiTS on all host threads)
 on the same workload; rank 0 only.
+
+--dump-outputs DIR writes the float32 RGBA image of the last timed step (1280x720x4; at N > 1 the assembled image)
+to DIR/image.npy from rank 0. Which frames that step renders depends only on W (at least 3), K and N, so two builds
+run with the same arguments can be compared image for image. At N = 1 it is frame W+K-1 alone, which --mode exact and
+--impl reference render bit for bit like the reference; the fast mode adds its samples with float atomics, so two of
+its runs agree to rounding, not bit for bit.
 """
 import argparse
 import json
@@ -103,6 +109,12 @@ class ClockSampler:
                 "reasons": reasons, "samples": len(sm)}
 
 
+def dump_outputs(directory, **arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def run_reference(args, rank):
     """The reference's own CPU implementation on the host cores (its enkiTS scheduler uses every hardware thread,
     Cpp/Source/enkiTS/TaskScheduler.cpp:1301). One step = one 1280x720 4-spp frame, like ours."""
@@ -122,6 +134,8 @@ def run_reference(args, rank):
         render = lambda f0, n: (lambda r: (r[1], r[3]))(pyoracle.orc_render(sph, mats, cam, W, H, f0, n, flags=0, buf=buf, want_seconds=True))
     render(0, max(2, args.warmup))            # first frames pay thread spin-up (SURVEY §6)
     rays, secs = render(args.warmup, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, image=buf)
     total_s = sum(secs)
     value = sum(rays) / total_s / 1e6
     line = {"impl": "reference", "metric": "Mray/s on 46-sphere scene @1280x720", "value": value, "unit": "Mray/s",
@@ -209,6 +223,7 @@ def main():
     ap.add_argument("--variant", type=int, default=-1, help="fast kernel variant (default: library default)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-strong", action="store_true", help="skip the 3840x2160x64spp strong-scaling sub-record (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's image as DIR/image.npy (float32)")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -292,6 +307,8 @@ def main():
     barrier()
     wall = time.perf_counter() - wall0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, image=(image if world == 1 else assembled[0]).cpu().numpy())
     step_ms = [a.elapsed_time(c) for a, b, c in evs]
     kernel_step_ms = [a.elapsed_time(b) for a, b, c in evs]
     exchange_ms = [b.elapsed_time(c) for a, b, c in evs]

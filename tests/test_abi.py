@@ -8,7 +8,7 @@ import re
 import numpy as np
 import pytest
 
-from test_oracle import golden_scene
+from test_oracle import golden_scene, parity_scene
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -42,12 +42,9 @@ def test_shim_scene_equals_reference_export(libs):
     assert list(em) == list(ge) == [8, 45]
 
 
-def test_shim_camera_and_animation_equal_reference(libs, oracle):
-    if not oracle.have_ref():
-        pytest.skip("needs the reference")
+def test_shim_camera_and_animation_equal_reference(libs):
     for (w, h, flags, t) in [(3840, 2160, 0, 0.0), (640, 480, 1, 1.25), (256, 144, 3, 7.5)]:
-        # animated calls leave the reference's static scene moved for the rest of its process: isolate them
-        rs, rm, rc, re_ = oracle.isolated("ref_scene", w, h, time=t, flags=flags)
+        rs, rm, rc, re_ = parity_scene(f"stock_{w}x{h}_t{t}_flags{flags}")
         sph, mats, cam, em = libs.reference_scene(w, h, time=t, flags=flags)
         assert sph.tobytes() == rs.tobytes() and mats.tobytes() == rm.tobytes() and cam.tobytes() == rc.tobytes()
         assert list(em) == list(re_)

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 from conftest import bits_differ
-from test_oracle import GOLD, golden_scene
+from test_oracle import GOLD, PARITY, assert_equals_reference, golden_scene
 
 pytestmark = pytest.mark.gpu
 
@@ -50,7 +50,7 @@ def test_golden_vectors(gpu_ctx):
     gpu_ctx.set_option("exact_lanes", 0)
 
 
-def test_dropin_drawtest_full_size_vs_golden_counts_and_reference(libs, oracle):
+def test_dropin_drawtest_full_size_vs_golden_counts_and_reference(libs):
     """The BASELINE configuration (46 spheres, 1280x720, 4 spp) through the drop-in's UpdateTest/DrawTest."""
     counts = json.load(open(os.path.join(GOLD, "ref_counts.json")))["1280x720_flags0_frames0-5"]
     w, h = 1280, 720
@@ -64,10 +64,7 @@ def test_dropin_drawtest_full_size_vs_golden_counts_and_reference(libs, oracle):
         rays.append(libs.DrawTest(0.0, f, w, h, buf, 0))
     assert rays == counts[:3]                                    # 16 809 105 / 16 822 947 / 16 818 090
     assert (buf[..., 3] == 0).all()                              # alpha untouched (Maths.h:38)
-    if oracle.have_ref():
-        rbuf, rrays = oracle.ref_render(w, h, 0, 3, flags=0)
-        assert rrays == rays
-        assert not bits_differ(buf, rbuf).any()
+    assert_equals_reference(buf, rays, [], "stock_1280x720_t0.0_flags0_frames0+3")
     libs.ShutdownTest()
 
 
@@ -149,7 +146,7 @@ def test_runtime_scenes_against_restatement(libs, gpu_ctx, oracle):
     gpu_ctx.set_option("exact_lanes", 0)
 
 
-def test_padded_sphere_hit_frame(gpu_ctx, oracle):
+def test_padded_sphere_hit_frame(gpu_ctx):
     """Frame 28 at 1280x720 holds a ray that hits a padded impossible sphere (reference UB): ray counts must still
     equal the reference's, and every pixel except that one must be bit-identical."""
     sph, mats, cam, em = golden_scene()
@@ -157,10 +154,7 @@ def test_padded_sphere_hit_frame(gpu_ctx, oracle):
     buf = np.zeros((720, 1280, 4), np.float32)
     rays = gpu_ctx.draw(28, 1, 1280, 720, buf, flags=0, mode=0)
     assert rays == 16813074
-    if oracle.have_ref():
-        rbuf, rrays = oracle.ref_render(1280, 720, 28, 1, flags=0)
-        assert rrays == [rays]
-        assert not bits_differ(buf, rbuf, [(180, 436, 28)]).any()
+    assert_equals_reference(buf, [rays], [(180, 436, 28)], "stock_1280x720_t0.0_flags0_frames28+1")
 
 
 def test_4k_frame_ray_count(gpu_ctx, libs):
@@ -176,21 +170,18 @@ def test_4k_frame_ray_count(gpu_ctx, libs):
 
 def test_headless_shell_same_output_as_reference_build(libs):
     """One shell source (toypathtracer_b200/csrc/headless_main.cpp, the shape of Cpp/Emscripten/main.cpp:46-61) built
-    twice — against the unmodified reference sources (oracle/_ref/ref_headless) and against the drop-in
-    (toypathtracer_b200/tpt_headless) — must print the same ray counts and the same backbuffer checksum."""
+    twice — against the unmodified reference sources (oracle/_ref/ref_headless, its output recorded in
+    tests/golden/ref_parity.json) and against the drop-in (toypathtracer_b200/tpt_headless) — must print the same ray
+    counts and the same backbuffer checksum."""
     import subprocess
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     ours = os.path.join(root, "toypathtracer_b200", "tpt_headless")
-    ref = os.path.join(root, "oracle", "_ref", "ref_headless")
-    if not (os.path.exists(ours) and os.path.exists(ref)):
-        pytest.skip("headless binaries not built")
-    args = ["384", "216", "4", "2"]
+    ref = PARITY["headless"]
     env = dict(os.environ, TPT_MODE="exact")
-    a = subprocess.run([ours] + args, capture_output=True, text=True, env=env, timeout=300)
-    b = subprocess.run([ref] + args, capture_output=True, text=True, timeout=300)
+    a = subprocess.run([ours] + ref["args"], capture_output=True, text=True, env=env, timeout=300)
     assert a.returncode == 0, a.stderr
     keep = lambda out: [l for l in out.splitlines() if l.startswith("frame") or l.startswith("checksum")]
-    assert keep(a.stdout) == keep(b.stdout) and len(keep(a.stdout)) == 5
+    assert keep(a.stdout) == ref["lines"] and len(ref["lines"]) == 5
 
 
 def test_odd_sizes_and_single_row(gpu_ctx, oracle):

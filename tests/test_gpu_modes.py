@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 
 from conftest import bits_differ, rel_l2
-from test_oracle import golden_scene
+from test_oracle import assert_equals_reference, golden_scene
 
 pytestmark = pytest.mark.gpu
 
@@ -28,10 +28,7 @@ def test_exact_mode_equals_reference_variant_build(gpu_ctx, libs, oracle, varian
                 total, pf = gpu_ctx.draw(0, 3, w, h, buf, flags=flags, mode=0, per_frame=True)
                 assert pf == orays, (variant, flags, lanes)
                 assert not bits_differ(buf, obuf, pads).any(), (variant, flags, lanes)
-            if oracle.have_ref_variant(variant):
-                rbuf, rrays = oracle.ref_render(w, h, 0, 3, flags=flags, variant=variant)
-                assert rrays == pf
-                assert not bits_differ(buf, rbuf, pads).any()
+            assert_equals_reference(buf, pf, pads, f"{variant}_{w}x{h}_t0.0_flags{flags}_frames0+3")
         # fast mode honours the switches too (statistically): 256 spp vs the restatement at 256 spp
         obuf, orays, _ = oracle.orc_render(sph, mats, cam, w, h, 0, 64, flags=2, mitsuba=mitsuba)
         o2 = obuf.copy()
@@ -48,8 +45,6 @@ def test_exact_mode_equals_reference_variant_build(gpu_ctx, libs, oracle, varian
 
 def test_dropin_shim_variants_through_drawtest(libs, oracle):
     """The Test.h drop-in with tpt_shim_set_variant(): UpdateTest/DrawTest of the 9-sphere Mitsuba-compare build."""
-    if not oracle.have_ref_variant("small_mitsuba"):
-        pytest.skip("reference variant not built")
     w, h = 256, 144
     libs.set_variant(False, True)
     try:
@@ -61,11 +56,9 @@ def test_dropin_shim_variants_through_drawtest(libs, oracle):
         for f in range(3):
             libs.UpdateTest(0.0, f, w, h, 2)
             rays.append(libs.DrawTest(0.0, f, w, h, buf, 2))
-        rbuf, rrays = oracle.ref_render(w, h, 0, 3, flags=2, variant="small_mitsuba")
         sph, mats, cam, em = libs.GetSceneDesc()
         _, _, pads = oracle.orc_render(sph, mats, cam, w, h, 0, 3, flags=2, mitsuba=True)
-        assert rays == rrays
-        assert not bits_differ(buf, rbuf, pads).any()
+        assert_equals_reference(buf, rays, pads, "small_mitsuba_256x144_t0.0_flags2_frames0+3")
         libs.ShutdownTest()
     finally:
         libs.set_variant(True, False)

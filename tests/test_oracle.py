@@ -1,5 +1,6 @@
 """Pins the oracle: the CPU restatement (oracle/restate.cpp) against the committed golden vectors generated from
-the unmodified reference, and against the reference itself where oracle/_ref/libtoyref.so is present."""
+the unmodified reference (tests/golden/make_golden.py, make_golden_parity.py)."""
+import hashlib
 import json
 import os
 
@@ -9,11 +10,40 @@ import pytest
 from conftest import bits_differ
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
+PARITY = json.load(open(os.path.join(GOLD, "ref_parity.json")))
 
 
 def golden_scene():
     g = np.load(os.path.join(GOLD, "scene46_1280x720.npz"))
     return g["spheres"], g["materials"].view(np.float32), g["camera"], g["emissives"]
+
+
+def parity_scene(key):
+    """The reference's GetSceneDesc export recorded under `key` (variant_WxH_tTIME_flagsFLAGS)."""
+    g = np.load(os.path.join(GOLD, "ref_parity_scenes.npz"))
+    return g[f"{key}/spheres"], g[f"{key}/materials"].view(np.float32), g[f"{key}/camera"], g[f"{key}/emissives"]
+
+
+def parity_render(key):
+    """The reference's render recorded under `key`: {"rays", "pads", "sha256_pads_zeroed"}."""
+    r = PARITY["renders"][key]
+    return dict(r, pads=[tuple(p) for p in r["pads"]])
+
+
+def image_hash(img, pads):
+    """sha256 of the float32 RGBA bytes with the padded-sphere pixels (x, y[, frame]) zeroed."""
+    img = np.array(img, np.float32, copy=True)
+    for p in pads:
+        img[p[1], p[0]] = 0
+    return hashlib.sha256(np.ascontiguousarray(img).tobytes()).hexdigest()
+
+
+def assert_equals_reference(buf, rays, pads, key):
+    """Ray counts, padded-sphere pixels and every other pixel's bits equal the reference's render `key`."""
+    g = parity_render(key)
+    assert rays == g["rays"], key
+    assert pads == g["pads"], key
+    assert image_hash(buf, pads) == g["sha256_pads_zeroed"], key
 
 
 def scene_for(oracle, w, h):
@@ -44,40 +74,31 @@ def test_golden_ray_counts_720p(oracle):
 
 
 def test_restatement_equals_reference_bitwise(oracle):
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref/libtoyref.so not built (reference sources absent)")
     for (w, h, f0, nf, flags) in [(320, 180, 0, 3, 2), (200, 120, 7, 2, 0)]:
-        sph, mats, cam, em = oracle.ref_scene(w, h)
-        rbuf, rrays = oracle.ref_render(w, h, f0, nf, flags=flags)
+        sph, mats, cam, em = parity_scene(f"stock_{w}x{h}_t0.0_flags{flags}")
         obuf, orays, pads = oracle.orc_render(sph, mats, cam, w, h, f0, nf, flags=flags)
-        assert orays == rrays
-        assert not bits_differ(obuf, rbuf, pads).any()
+        assert_equals_reference(obuf, orays, pads, f"stock_{w}x{h}_t0.0_flags{flags}_frames{f0}+{nf}")
 
 
 def test_restatement_equals_reference_animated(oracle):
     """kFlagAnimate: spheres 1 and 8 move with time, lerpFac *= 0.9 (Test.cpp:273-274,304-308)."""
-    if not oracle.have_ref():
-        pytest.skip("needs the reference")
     w, h, t, flags = 160, 90, 1.25, 3
-    sph, mats, cam, em = oracle.isolated("ref_scene", w, h, time=t, flags=flags)
-    rbuf, rrays = oracle.isolated("ref_render", w, h, 40, 2, flags=flags, time=t)
+    sph, mats, cam, em = parity_scene(f"stock_{w}x{h}_t{t}_flags{flags}")
     obuf, orays, pads = oracle.orc_render(sph, mats, cam, w, h, 40, 2, flags=flags)
-    assert orays == rrays
-    assert not bits_differ(obuf, rbuf, pads).any()
+    assert_equals_reference(obuf, orays, pads, f"stock_{w}x{h}_t{t}_flags{flags}_frames40+2")
 
 
 def test_padded_sphere_hit_control_flow(oracle):
     """Frame 28 of the 1280x720 sequence contains a path ray that 'hits' a padded impossible sphere (reference UB,
     see oracle/restate.cpp Trace()). The restatement must follow the reference's control flow: equal ray counts,
     and only that pixel may differ."""
-    if not oracle.have_ref():
-        pytest.skip("needs the reference")
-    sph, mats, cam, em = oracle.ref_scene(1280, 720)
-    rbuf, rrays = oracle.ref_render(1280, 720, 28, 1, flags=0)
+    sph, mats, cam, em = parity_scene("stock_1280x720_t0.0_flags0")
+    gs, gm, gc, ge = golden_scene()
+    assert sph.tobytes() == gs.tobytes() and mats.tobytes() == gm.tobytes() and cam.tobytes() == gc.tobytes()
     obuf, orays, pads = oracle.orc_render(sph, mats, cam, 1280, 720, 28, 1, flags=0)
-    assert orays == rrays == [16813074]
+    assert orays == [16813074]
     assert pads == [(180, 436, 28)]
-    assert not bits_differ(obuf, rbuf, pads).any()
+    assert_equals_reference(obuf, orays, pads, "stock_1280x720_t0.0_flags0_frames28+1")
 
 
 def test_scalar_vs_simd_tie_rule_agree_on_reference_scene(oracle):
@@ -104,20 +125,16 @@ def test_runtime_scene_edge_cases(oracle):
 def test_reference_compile_time_variants(oracle, variant, big, mitsuba):
     """DO_MITSUBA_COMPARE (Config.h:25) and DO_BIG_SCENE 0 (Test.cpp:10-11): the reference compiled from an edited
     temporary copy (oracle/Makefile) vs the restatement's runtime switch and the drop-in shim's scene export."""
-    if not oracle.have_ref_variant(variant):
-        pytest.skip(f"oracle/_ref/libtoyref_{variant}.so not built (reference sources absent)")
     import toypathtracer_b200 as tpt
     w, h = 200, 120
-    sph, mats, cam, em = oracle.ref_scene(w, h, variant=variant)
-    assert len(sph) == (46 if big else 9)
-    s2, m2, c2, e2 = tpt.reference_scene(w, h, big_scene=big, mitsuba_compare=mitsuba)      # the shim's UpdateTest/GetSceneDesc
-    assert s2.tobytes() == sph.tobytes() and m2.tobytes() == mats.tobytes() and c2.tobytes() == cam.tobytes()
-    assert list(e2) == list(em)
     for flags in (0, 2):
-        rbuf, rrays = oracle.ref_render(w, h, 0, 3, flags=flags, variant=variant)
+        sph, mats, cam, em = parity_scene(f"{variant}_{w}x{h}_t0.0_flags{flags}")
+        assert len(sph) == (46 if big else 9)
+        s2, m2, c2, e2 = tpt.reference_scene(w, h, big_scene=big, mitsuba_compare=mitsuba)      # the shim's UpdateTest/GetSceneDesc
+        assert s2.tobytes() == sph.tobytes() and m2.tobytes() == mats.tobytes() and c2.tobytes() == cam.tobytes()
+        assert list(e2) == list(em)
         obuf, orays, pads = oracle.orc_render(sph, mats, cam, w, h, 0, 3, flags=flags, mitsuba=mitsuba)
-        assert orays == rrays
-        assert not bits_differ(obuf, rbuf, pads).any()
+        assert_equals_reference(obuf, orays, pads, f"{variant}_{w}x{h}_t0.0_flags{flags}_frames0+3")
 
 
 def test_refgpu_oracle_is_the_same_estimator_statistically(oracle):
